@@ -52,12 +52,13 @@ def log(*a):
 # ------------------------------------------------------------------------------------------------------------------
 # workload synthesis (never timed)
 # ------------------------------------------------------------------------------------------------------------------
-def make_workload(name: str, rank: int, clips_override: int | None, world: int = 1):
+def make_workload(name: str, rank: int, clips_override: int | None, world: int = 1, replicated: bool = False):
+    """`replicated`: the committed golden clip even when the reference compressor is available (the request list is the same)."""
     kind, num_clips, bones, samples, description = WORKLOADS[name]
     if clips_override:
         num_clips = clips_override
     from oracle import ref
-    distinct = ref.available()
+    distinct = ref.available() and not replicated
     if kind == "transform":
         if distinct:
             spec = ref.TransformSpec(num_tracks=bones, num_samples=samples, seed={"c2": 2000, "c3": 3000, "c5": 5000}[name] + rank * num_clips)
@@ -359,6 +360,26 @@ def workload_config(args, w, world: int, num_requests: int, pose_bytes: int, blo
             "math": MATH_DESCRIPTION[args.math if is_transform else "exact"], "parallelism": f"clip-sharded x{world}, no data-path collective"}
 
 
+DUMP_BYTES = 32 << 20      # --dump-outputs budget, shared by the ranks
+DUMP_SEED = 0
+
+
+def dump_outputs(directory: str, d_out, num_requests: int, max_tracks: int, bone_bytes: int, rank: int, world: int) -> None:
+    """Writes the poses of a fixed, seeded sample of this rank's requests (all of them when they fit its DUMP_BYTES / world share) in request order:
+    float32 [requests][max_tracks][bone_bytes / 4], the layout the caller's output buffer holds."""
+    import torch
+    lanes = bone_bytes // 4
+    poses = d_out.view(torch.float32).view(num_requests, max_tracks, lanes)
+    keep = min(num_requests, max(1, DUMP_BYTES // world // (max_tracks * bone_bytes)))
+    if keep < num_requests:
+        pick = np.sort(np.random.default_rng(DUMP_SEED).choice(num_requests, size=keep, replace=False))
+        poses = poses.index_select(0, torch.from_numpy(pick).to(poses.device))
+    os.makedirs(directory, exist_ok=True)
+    name = "poses.npy" if world == 1 else f"poses.rank{rank}.npy"
+    np.save(os.path.join(directory, name), poses.cpu().numpy())
+    log(f"[bench] wrote {keep} of {num_requests} requests' poses to {os.path.join(directory, name)}")
+
+
 def time_launches(torch, launch, stream, steps: int, warmup: int, barrier, sampler=None):
     """W untimed + K timed launches bracketed by barrier + synchronize; returns (elapsed ms of the K steps, median launch ms)."""
     for _ in range(warmup):
@@ -395,7 +416,9 @@ def measured_traffic(workload: str):
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed launches of every timed loop (headline, other math mode, e2e, extra workloads, routed C5 job); the per workload "
+                         "clock records poll NVML every 1 ms, so a fast workload needs enough steps to span a few ms or it reports no samples")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=list(WORKLOADS))
@@ -409,6 +432,9 @@ def main() -> None:
     ap.add_argument("--gather", action="store_true", help="N > 1: also time decode + NCCL all-gather of the poses (SURVEY 8e, optional consumer-side gather)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra blocks (other workloads at N = 1, the routed C5 job at N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the poses the last timed step produced (a fixed sample of the requests, at most "
+                         f"{DUMP_BYTES >> 20} MB over all ranks) as DIR/poses.npy (poses.rank<r>.npy with N > 1), float32 [requests][tracks][lanes], to compare two builds output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -475,7 +501,8 @@ def main() -> None:
     bone_bytes = (40 if layout == ab.LAYOUT_QVV40 else 48) if is_transform else 4 * clipset.components
     pose_bytes = clipset.max_tracks * bone_bytes
     d_requests = torch.from_numpy(requests.view(np.uint8)).cuda()
-    d_out = torch.empty(num_requests * pose_bytes, dtype=torch.uint8, device="cuda")
+    # zeroed when dumped: lanes the layout leaves unwritten must not carry whatever the allocator held
+    d_out = (torch.zeros if args.dump_outputs else torch.empty)(num_requests * pose_bytes, dtype=torch.uint8, device="cuda")
     stream = torch.cuda.current_stream()
 
     def launch():
@@ -499,6 +526,8 @@ def main() -> None:
     launches_before = ctx.launch_count
     rank_ms, kernel_ms = time_launches(torch, launch, stream, args.steps, args.warmup, barrier, sampler)
     clocks = sampler.stop()
+    if args.dump_outputs:       # before the other arithmetic mode and the e2e path overwrite the buffer
+        dump_outputs(args.dump_outputs, d_out, num_requests, clipset.max_tracks, bone_bytes, rank, world)
     gpu_launches = ctx.launch_count - launches_before - args.warmup
     elapsed_ms = reducer.max(rank_ms)                                   # slowest rank
     value = reducer.sum(units_per_step * args.steps) / (elapsed_ms * 1e-3)   # every rank's units
@@ -540,7 +569,7 @@ def main() -> None:
         h_out = torch.empty(num_requests * pose_bytes, dtype=torch.uint8).pin_memory()
         req_np = h_requests.numpy().view(ab.api.REQUEST_DTYPE)
         out_np = h_out.numpy()
-        e2e_steps = max(args.steps, 2)
+        e2e_steps = args.steps
         for _ in range(2):
             ctx.decompress_tracks_host(clipset, req_np, options, out_np)     # warm-up (allocates the device scratch)
         barrier()
@@ -608,10 +637,10 @@ def main() -> None:
         del d_out
         workloads = {}
         for name in ("c3", "c5", "c4"):
-            workloads[name] = extra_workload(name, torch, ab, ctx, local_rank, peak, barrier)
+            workloads[name] = extra_workload(name, torch, ab, ctx, local_rank, peak, barrier, args.steps)
         if w["distinct"]:
             try:
-                workloads["error_metric"] = error_metric_workload(torch, ab, ctx, w, clipset, local_rank, peak, barrier)
+                workloads["error_metric"] = error_metric_workload(torch, ab, ctx, w, clipset, local_rank, peak, barrier, args.steps)
             except Exception as failure:      # an extra block must not take the headline line down with it; it is reported, not hidden
                 workloads["error_metric"] = {"failed": f"{type(failure).__name__}: {failure}"}
 
@@ -638,9 +667,8 @@ def sample_single_thread(w, blobs) -> float:
     return sample * w["num_tracks"] / seconds
 
 
-def extra_workload(name: str, torch, ab, ctx, local_rank: int, peak: float, barrier) -> dict:
-    """One of the other configs on the same GPU: a short timed run with its own clock record (steps sized so that the NVML poll
-    gets samples inside the region)."""
+def extra_workload(name: str, torch, ab, ctx, local_rank: int, peak: float, barrier, steps: int) -> dict:
+    """One of the other configs on the same GPU: `steps` timed launches with their own clock record."""
     w = make_workload(name, 0, None)
     is_transform = w["kind"] == "transform"
     clipset = ctx.upload_packed(w["buffer"], w["offsets"], w["sizes"])
@@ -660,12 +688,6 @@ def extra_workload(name: str, torch, ab, ctx, local_rank: int, peak: float, barr
     alg = algorithmic_bytes_transform(w) if is_transform else algorithmic_bytes_scalar(w)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    for _ in range(3):
-        launch()
-    torch.cuda.synchronize()
-    probe0, probe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    probe0.record(stream); launch(); probe1.record(stream); torch.cuda.synchronize()
-    steps = int(min(400, max(20, 40.0 / max(probe0.elapsed_time(probe1), 1e-3))))       # about 40 ms of launches: tens of clock samples
     elapsed_ms, kernel_ms = time_launches(torch, launch, stream, steps, 3, barrier, sampler)
     clocks = sampler.stop()
     achieved = alg["total"] / (kernel_ms * 1e-3) / 1e9
@@ -677,7 +699,7 @@ def extra_workload(name: str, torch, ab, ctx, local_rank: int, peak: float, barr
     return out
 
 
-def error_metric_workload(torch, ab, ctx, w, clipset, local_rank: int, peak: float, barrier, num_clips: int = 4096) -> dict:
+def error_metric_workload(torch, ab, ctx, w, clipset, local_rank: int, peak: float, barrier, steps: int, num_clips: int = 4096) -> dict:
     """SURVEY 8(f1): acl::calculate_compression_error (decode every sample of a clip, object space, qvvf_transform_error_metric against the
     raw poses, worst track) for the first `num_clips` clips of the C2 clip set in ONE call, poses never leaving the GPU. Unit: bone-poses
     MEASURED per second. The CPU figure next to it is the unmodified reference's calculate_compression_error on a bounded sample."""
@@ -712,9 +734,6 @@ def error_metric_workload(torch, ab, ctx, w, clipset, local_rank: int, peak: flo
     launch()
     launches_per_call = ctx.launch_count - launches_before
     torch.cuda.synchronize()
-    probe0, probe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    probe0.record(stream); launch(); probe1.record(stream); torch.cuda.synchronize()
-    steps = int(min(200, max(10, 60.0 / max(probe0.elapsed_time(probe1), 1e-3))))
     elapsed_ms, call_ms = time_launches(torch, launch, stream, steps, 3, barrier, sampler)
     clocks = sampler.stop()
     errors = d_errors.cpu().numpy().view(ab.TRACK_ERROR_DTYPE)
@@ -800,7 +819,7 @@ def routed_c5_job(args, torch, dist, ab, ctx, rank, local_rank, world, reducer, 
     stream = torch.cuda.current_stream()
     sampler = ClockSampler(local_rank)
     sampler.start()
-    steps = 200
+    steps = args.steps
     rank_ms, kernel_ms = time_launches(torch, lambda: ctx.decompress_tracks(clipset, d_requests, n, options, d_out, stream), stream, steps, 5, barrier, sampler)
     clocks = sampler.stop()
     elapsed_ms = reducer.max(rank_ms)

@@ -10,6 +10,7 @@ key frame stripping) and the edge cases its validation walks (tools/acl_compress
 """
 from __future__ import annotations
 
+import hashlib
 import os
 
 import numpy as np
@@ -90,3 +91,22 @@ def sample_times(spec) -> np.ndarray:
 
 def bit_equal(a: np.ndarray, b: np.ndarray) -> bool:
     return np.array_equal(np.ascontiguousarray(a, dtype=np.float32).view(np.uint32), np.ascontiguousarray(b, dtype=np.float32).view(np.uint32))
+
+
+def digest(*arrays: np.ndarray) -> int:
+    """64 bit BLAKE2b of the bytes of `arrays` (floats as float32), in order: two digests are equal exactly when every bit is (a
+    chance collision aside), so a stored digest of the reference's output stands for the output in a bit for bit comparison."""
+    h = hashlib.blake2b(digest_size=8)
+    for a in arrays:
+        a = np.asarray(a)
+        h.update(np.ascontiguousarray(a, dtype=np.float32 if a.dtype.kind == "f" else a.dtype).tobytes())
+    return int.from_bytes(h.digest(), "little")
+
+
+REFERENCE_CHECKS = os.path.join(GOLDEN_DIR, "reference_checks.npz")
+
+
+def reference_checks(key: str) -> np.ndarray:
+    """What the reference computed for the comparison `key` (tests/golden/make_reference_checks.py)."""
+    with np.load(REFERENCE_CHECKS) as stored:
+        return stored[key]
